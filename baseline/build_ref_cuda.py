@@ -17,17 +17,13 @@ The module is built under the name `inference_extensions_cuda_ref` (pybind's TOR
 one process with the product's `inference_extensions_cuda` package; `load_as_plugin()` installs it in sys.modules under the
 reference's own name for the processes that drive the unmodified reference models with the reference's kernels.
 
-Also emits sourceless byte-code of the reference's Python surface (src/, test_video.py, test_compress_time.py) into
-baseline/_ref/py/ — a build output like the .so, so that the *unmodified* reference models / drivers can be imported on
-the GPU box (which has no /root/reference).  No reference source text is copied into the repository.
+The reference's Python surface that drives it is the byte-code oracle/build_ref.py emits into oracle/_ref/py.
 """
 from __future__ import annotations
 
 import glob
 import importlib.util
 import os
-import py_compile
-import shutil
 import subprocess
 import sys
 import sysconfig
@@ -38,7 +34,6 @@ EXT = os.path.join(REF, "src/layers/extensions/inference")
 RANS = os.path.join(REF, "src/cpp/py_rans")
 OUT = os.path.join(HERE, "_ref")
 OBJ = os.path.join(OUT, "obj")
-PY_OUT = os.path.join(OUT, "py")
 MODNAME = "inference_extensions_cuda_ref"
 
 
@@ -107,27 +102,6 @@ def write_ninja(jobs_split: int = 2) -> str:
     return path
 
 
-def build_py_surface() -> str | None:
-    """Sourceless byte-code of the reference's Python surface -> baseline/_ref/py (importable on the GPU box)."""
-    if not os.path.isdir(REF):
-        return PY_OUT if os.path.isdir(PY_OUT) else None
-    files = [os.path.join(REF, "test_video.py"), os.path.join(REF, "test_compress_time.py")]
-    files += sorted(glob.glob(os.path.join(REF, "src/**/*.py"), recursive=True))
-    for f in files:
-        rel = os.path.relpath(f, REF)
-        if rel.startswith("src/cpp") or "extensions" in rel and rel.endswith("setup.py"):
-            continue
-        dst = os.path.join(PY_OUT, rel + "c")
-        os.makedirs(os.path.dirname(dst), exist_ok=True)
-        if not os.path.exists(dst) or os.path.getmtime(dst) < os.path.getmtime(f):
-            py_compile.compile(f, cfile=dst, dfile=rel, doraise=True)
-    # the reference's test configuration (JSON, data not code) is read by test_video.py at run time
-    cfg_src, cfg_dst = os.path.join(REF, "test_cfg"), os.path.join(PY_OUT, "test_cfg")
-    if os.path.isdir(cfg_src) and not os.path.isdir(cfg_dst):
-        shutil.copytree(cfg_src, cfg_dst)
-    return PY_OUT
-
-
 def build_ref_cuda(force: bool = False, jobs: int | None = None) -> str | None:
     """Returns the path of the built module; None if the reference tree is absent and nothing is prebuilt."""
     out = module_path()
@@ -160,5 +134,4 @@ def load(as_plugin: bool = False):
 
 
 if __name__ == "__main__":
-    print("[baseline] py surface:", build_py_surface())
     print("[baseline] reference CUDA extension:", build_ref_cuda(force="--force" in sys.argv))

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Times the REFERENCE's own CUDA path on this box: the reference's unmodified Python models (src/models, from
-/root/reference or the byte-code in baseline/_ref/py) on top of the reference's own CUTLASS extension compiled for sm_100a
+"""Times the REFERENCE's own CUDA path on this box: the reference's unmodified Python models (src/models, the
+byte-code in oracle/_ref/py) on top of the reference's own CUTLASS extension compiled for sm_100a
 (baseline/build_ref_cuda.py -> baseline/_ref/inference_extensions_cuda_ref*.so) — none of this repository's kernels on the
 path.  Same synthetic checkpoints, frames, q_index, skip_thres and timing protocol as bench.py's product arm (CUDA events
 per call, L2 flushed between calls; test_video.py:204-325 times one call at a time the same way).
@@ -44,7 +44,11 @@ def main():
     if ext is None:
         print(json.dumps({"unavailable": "baseline/_ref/inference_extensions_cuda_ref*.so not built"}))
         return
-    ref_root = "/root/reference" if os.path.isdir("/root/reference/src/models") else os.path.join(ROOT, "baseline", "_ref", "py")
+    from oracle.build_ref import py_surface_root
+    ref_root = py_surface_root()
+    if ref_root is None:
+        print(json.dumps({"unavailable": "oracle/_ref/py (the reference's models as byte-code) not built"}))
+        return
     sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))   # MLCodec_extensions_cpp (the reference's rANS module)
     sys.path.insert(0, ref_root)
     from src.models.image_model import DMCI

@@ -5,17 +5,27 @@ streams are bit-identical to the reference's.  Reference sources are never copie
 
 The reference's own build (src/cpp/setup.py) is a 3-file pybind11 extension; we invoke g++ on
 those files directly.
+
+Also emits sourceless byte-code of the reference's Python surface (src/, test_video.py,
+test_compress_time.py) into oracle/_ref/py: a build output like the .so, so that the tests can import
+the *unmodified* reference models on a machine without the reference tree.  No reference source text
+is copied into the repository.
 """
 from __future__ import annotations
 
+import glob
 import os
+import py_compile
+import shutil
 import subprocess
 import sys
 import sysconfig
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = "/root/reference/src/cpp/py_rans"
+REF = "/root/reference"
+REF_SRC = os.path.join(REF, "src/cpp/py_rans")
 OUT_DIR = os.path.join(HERE, "_ref")
+PY_OUT = os.path.join(OUT_DIR, "py")
 
 
 def ref_module_path() -> str:
@@ -61,6 +71,33 @@ def build_ref(force: bool = False) -> str | None:
     return out
 
 
+def build_py_surface() -> str | None:
+    """Sourceless byte-code of the reference's Python surface -> oracle/_ref/py.  Returns that directory, or None
+    if the reference tree is absent and nothing is prebuilt."""
+    if not os.path.isdir(REF):
+        return PY_OUT if os.path.isdir(PY_OUT) else None
+    files = [os.path.join(REF, "test_video.py"), os.path.join(REF, "test_compress_time.py")]
+    files += sorted(glob.glob(os.path.join(REF, "src/**/*.py"), recursive=True))
+    for f in files:
+        rel = os.path.relpath(f, REF)
+        if rel.startswith("src/cpp") or "extensions" in rel and rel.endswith("setup.py"):
+            continue
+        dst = os.path.join(PY_OUT, rel + "c")
+        os.makedirs(os.path.dirname(dst), exist_ok=True)
+        if not os.path.exists(dst) or os.path.getmtime(dst) < os.path.getmtime(f):
+            py_compile.compile(f, cfile=dst, dfile=rel, doraise=True)
+    # the reference's test configuration (JSON, data not code) is read by test_video.py at run time
+    cfg_src, cfg_dst = os.path.join(REF, "test_cfg"), os.path.join(PY_OUT, "test_cfg")
+    if os.path.isdir(cfg_src) and not os.path.isdir(cfg_dst):
+        shutil.copytree(cfg_src, cfg_dst)
+    return PY_OUT
+
+
+def py_surface_root() -> str | None:
+    """oracle/_ref/py when it holds the reference's models (for sys.path), else None."""
+    return PY_OUT if os.path.isdir(os.path.join(PY_OUT, "src", "models")) else None
+
+
 def import_ref():
     """import MLCodec_extensions_cpp from oracle/_ref (None if unavailable)."""
     p = build_ref()
@@ -85,3 +122,4 @@ def import_ref_shim():
 
 if __name__ == "__main__":
     print(build_ref(force="--force" in sys.argv))
+    print(build_py_surface())

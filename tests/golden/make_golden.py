@@ -128,11 +128,51 @@ def make_stream():
         json.dump({"ops": ops, "length": len(data), "sha256": hashlib.sha256(data).hexdigest(), "head_hex": data[:512].hex()}, out)
 
 
+def container_random_ops(seed=11):
+    """random container writes (ids 0..15, heights / widths / payloads across the varint widths), same format as
+    container_script"""
+    rng = np.random.default_rng(seed)
+    ops = []
+    for i in range(16):
+        ops.append(["sps", i, int(rng.integers(1, 1 << 14)), int(rng.integers(1, 1 << 20))])
+        ops.append(["ip", bool(i & 1), i, int(rng.integers(0, 256)), int(rng.integers(0, 128)), int(rng.integers(0, 2)),
+                    int(rng.integers(0, 40000)), i])
+    return ops
+
+
+UINT_ADAPTIVE_VALUES = (0, 1, 127, 128, 16383, 16384, (1 << 30) - 1)
+
+
+def make_stream_random():
+    """the reference's container helpers on container_random_ops(11): stream length / sha256, and the bytes of
+    write_uint_adaptive for values on the varint boundaries"""
+    import hashlib
+    import io
+    from src.utils.stream_helper import write_ip, write_sps, write_uint_adaptive  # reference
+    ops = container_random_ops(11)
+    f = io.BytesIO()
+    for op in ops:
+        if op[0] == "sps":
+            write_sps(f, {"sps_id": op[1], "height": op[2], "width": op[3]})
+        else:
+            write_ip(f, op[1], op[2], op[3], op[4], op[5], container_payload(op[6], op[7]))
+    data = f.getvalue()
+    uint = {}
+    for v in UINT_ADAPTIVE_VALUES:
+        b = io.BytesIO()
+        n = write_uint_adaptive(b, v)
+        uint[str(v)] = {"returned": n, "hex": b.getvalue().hex()}
+    with open(os.path.join(HERE, "stream_container_random.json"), "w") as out:
+        json.dump({"ops": ops, "length": len(data), "sha256": hashlib.sha256(data).hexdigest(),
+                   "uint_adaptive": uint}, out)
+
+
 def main():
     torch.manual_seed(0)
     torch.set_num_threads(8)
-    if "--only-stream" in sys.argv:   # adds the bitstream-container fixture without regenerating the others
+    if "--only-stream" in sys.argv:   # adds the bitstream-container fixtures without regenerating the others
         make_stream()
+        make_stream_random()
         print("container golden fixture written to", HERE)
         return
     if "--only-htl" in sys.argv:   # adds the HT-L fixtures without regenerating the others

@@ -164,17 +164,16 @@ def test_dcb_tail_declines_unsupported_shapes():
 
 
 def _reference_layers():
-    """the reference's own src/layers/layers.py (from /root/reference, or the byte-code in baseline/_ref/py on the GPU box)"""
-    import os
+    """the reference's own src/layers/layers.py (the byte-code oracle/build_ref.py emits into oracle/_ref/py)"""
     import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    for cand in ("/root/reference", os.path.join(root, "baseline", "_ref", "py")):
-        if os.path.isdir(os.path.join(cand, "src", "layers")):
-            if cand not in sys.path:
-                sys.path.insert(0, cand)
-            from src.layers import layers
-            return layers
-    return None
+    from oracle.build_ref import py_surface_root
+    root = py_surface_root()
+    if root is None:
+        return None
+    if root not in sys.path:
+        sys.path.insert(0, root)
+    from src.layers import layers
+    return layers
 
 
 @pytest.mark.parametrize("H,W,C,dcb2,shortcut", [(68, 120, 384, False, False), (136, 240, 384, False, True), (68, 120, 512, True, False)])

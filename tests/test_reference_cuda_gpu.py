@@ -3,10 +3,11 @@ identical inputs within 1e-3 PSNR / 1e-4 bpp").
 
 The reference's own CUTLASS extension, compiled for sm_100a by baseline/build_ref_cuda.py (un-modified sources, CUTLASS
 4.5.0 instead of the pinned 4.4.1), runs the reference's own models in a separate process (baseline/run_ref_cuda.py) on
-the synthetic checkpoints / frames of bench.py and dumps its streams and reconstructions; this process runs the product
-on the same inputs.  Both paths compute in fp16 with different accumulation (reference: fp16 accumulate in its CUTLASS
-epilogues and fp16 bias folds; here: fp32 accumulate, one rounding per op), so latents can differ by an fp16 ulp and a
-small fraction of quantisation ties flip.  The test measures that divergence (printed, and returned in bench.py's
+the synthetic checkpoints / frames of bench.py.  Its stream sizes and PSNRs on these inputs, measured on a B200, are stored
+in tests/golden/reference_cuda_parity.json and compared with on every run; where the extension is built, the run is also
+repeated live and the two reconstructions are compared with each other.  Both paths compute in fp16 with different
+accumulation (reference: fp16 accumulate in its CUTLASS epilogues and fp16 bias folds; here: fp32 accumulate, one rounding
+per op), so latents can differ by an fp16 ulp and a small fraction of quantisation ties flip.  The test measures that divergence (printed, and returned in bench.py's
 "parity" object) and asserts the contract's numbers where they hold and the measured bound x 2 where they do not.
 """
 import json
@@ -32,7 +33,7 @@ def _ref_built():
     return os.path.exists(build_ref_cuda.module_path())
 
 
-needs_ref = pytest.mark.skipif(not _ref_built(), reason="reference CUDA extension not built (python baseline/build_ref_cuda.py)")
+GOLDEN = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_cuda_parity.json")))
 
 
 def _run_ref(tmp, size, qp, models):
@@ -45,11 +46,10 @@ def _run_ref(tmp, size, qp, models):
     return info, np.load(os.path.join(tmp, f"ref_cuda_{size}_q{qp}.npz"))
 
 
-@needs_ref
 @pytest.mark.parametrize("size,qp", [("256x256", 32), ("1080x1920", 32), ("1080x1920", 0), ("1080x1920", 63)])
 def test_intra_against_reference_cuda(tmp_path, size, qp):
     h, w = (int(v) for v in size.split("x"))
-    info, dump = _run_ref(str(tmp_path), size, qp, "intra")
+    gold = GOLDEN["intra"][f"{size}_q{qp}"]
     from dcvc_b200.model import DMCI
     m = DMCI.synthetic(0)
     m.update(SKIP)
@@ -59,31 +59,32 @@ def test_intra_against_reference_cuda(tmp_path, size, qp):
     enc = m.compress(x, qp, pad_b, pad_r)
     ours = enc["x_hat"].float().cpu()[:, :, :h, :w]
     torch.cuda.synchronize()
-    ref = torch.from_numpy(dump["intra_x_hat"].astype(np.float32))
-    n_ref, n_ours = int(dump["intra_stream"].size), len(enc["bit_stream"])
+    n_ref, n_ours = gold["bytes"], len(enc["bit_stream"])
     d_bpp = abs(n_ours - n_ref) * 8 / (h * w)
-    p_ours, p_ref = psnr(ours, x.float().cpu()), psnr(ref, x.float().cpu())
-    cross = psnr(ours, ref)
-    same = bool(n_ours == n_ref and np.array_equal(np.frombuffer(enc["bit_stream"], dtype=np.uint8), dump["intra_stream"]))
-    print(f"[parity vs reference CUDA] intra {size} q{qp}: bytes {n_ours} vs {n_ref} (identical stream: {same}), "
-          f"d_bpp {d_bpp:.2e}, PSNR {p_ours:.4f} vs {p_ref:.4f} dB (d {abs(p_ours - p_ref):.2e}), "
-          f"PSNR(ours, ref) {cross:.2f} dB, max|dx| {(ours - ref).abs().max().item():.4f}")
-    assert info["intra"]["decode_equals_encode"]
+    p_ours, p_ref = psnr(ours, x.float().cpu()), gold["psnr_db"]
+    print(f"[parity vs reference CUDA] intra {size} q{qp}: bytes {n_ours} vs {n_ref}, "
+          f"d_bpp {d_bpp:.2e}, PSNR {p_ours:.4f} vs {p_ref:.4f} dB (d {abs(p_ours - p_ref):.2e})")
+    if _ref_built():
+        info, dump = _run_ref(str(tmp_path), size, qp, "intra")
+        ref = torch.from_numpy(dump["intra_x_hat"].astype(np.float32))
+        assert int(dump["intra_stream"].size) == n_ref and round(psnr(ref, x.float().cpu()), 4) == p_ref
+        cross = psnr(ours, ref)
+        print(f"[parity vs reference CUDA, live] PSNR(ours, ref) {cross:.2f} dB, max|dx| {(ours - ref).abs().max().item():.4f}")
+        assert info["intra"]["decode_equals_encode"]
+        assert cross >= 35.0   # the flipped ties move single latents by one quantisation step: local, bounded differences
     # The contract (BASELINE.json north_star): 1e-3 dB PSNR, 1e-4 bpp.  Measured on B200 (round 2,
     # profiles/r2_parity_vs_reference_cuda.md): PSNR within 1.3e-4 dB everywhere — asserted at the contract's 1e-3;
     # rate within 0.5e-4 .. 2.4e-4 bpp at 1080p (36 .. 62 bytes of 150 .. 440 KB: quantisation ties that flip between fp16-
     # and fp32-accumulated latents) — asserted at the measured bound x 2; a 256x256 frame has 7.5 KB, 10 bytes are 1.2e-3 bpp.
     assert abs(p_ours - p_ref) <= 1e-3
     assert d_bpp <= (5e-4 if h * w >= 1080 * 1920 else 2.5e-3)
-    assert cross >= 35.0   # the flipped ties move single latents by one quantisation step: local, bounded differences
 
 
-@needs_ref
 @pytest.mark.parametrize("name", ["hts", "ld", "htl"])
 def test_video_against_reference_cuda(tmp_path, name):
     size, qp = "256x384", 32
     h, w = 256, 384
-    info, dump = _run_ref(str(tmp_path), size, qp, name)
+    gold = GOLDEN["video_256x384_q32"][name]
     from dcvc_b200 import model as mm
     i_net = mm.DMCI.synthetic(0)
     i_net.update(SKIP)
@@ -106,13 +107,17 @@ def test_video_against_reference_cuda(tmp_path, name):
     d0 = p_net.decompress(e0["bit_stream"], {"height": h, "width": w}, qp, e0["ec_parallel"], 0)["x_hat"]
     d0 = d0[0] if isinstance(d0, list) else d0
     ours = d0.float().cpu()[:, :, :h, :w]
-    ref = torch.from_numpy(dump[name + "_x_hat0"].astype(np.float32))
-    n_ref, n_ours = int(dump[name + "_stream_sizes"][0]), len(e0["bit_stream"])
+    n_ref, n_ours = gold["bytes"], len(e0["bit_stream"])
     src = u0[:, :3].float().cpu()
-    p_ours, p_ref = psnr(ours, src), psnr(ref, src)
+    p_ours, p_ref = psnr(ours, src), gold["psnr_db"]
     d_bpp = abs(n_ours - n_ref) * 8 / (h * w * nf)
     print(f"[parity vs reference CUDA] {name} {size} q{qp} unit 0: bytes {n_ours} vs {n_ref}, d_bpp {d_bpp:.2e}, "
-          f"PSNR frame0 {p_ours:.4f} vs {p_ref:.4f} dB, PSNR(ours, ref) {psnr(ours, ref):.2f} dB")
+          f"PSNR frame0 {p_ours:.4f} vs {p_ref:.4f} dB")
+    if _ref_built():
+        _, dump = _run_ref(str(tmp_path), size, qp, name)
+        ref = torch.from_numpy(dump[name + "_x_hat0"].astype(np.float32))
+        assert int(dump[name + "_stream_sizes"][0]) == n_ref and round(psnr(ref, src), 4) == p_ref
+        print(f"[parity vs reference CUDA, live] PSNR(ours, ref) {psnr(ours, ref):.2f} dB")
     # measured (round 2): d_bpp 0.8e-4 (HT-S, LD) and 2.2e-4 (HT-L) at 256x384, PSNR within 1e-3 dB
     assert abs(p_ours - p_ref) <= 2e-3
     assert d_bpp <= 5e-4

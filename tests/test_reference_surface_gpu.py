@@ -3,9 +3,8 @@
 `north_star`: "keeping the src/models and src/layers Python operator API surface so test_video.py and
 test_compress_time.py run unmodified".  Here the reference's model classes (src/models/image_model.py:194-217,
 video_model_ht.py:413-450, video_model_ld.py:273-306) and its driver scripts (test_video.py:166-399,
-test_compress_time.py:23-69) are imported / executed as they are — from /root/reference where it exists (authoring
-container) or from the sourceless byte-code `baseline/build_ref_cuda.py` emits into baseline/_ref/py (the GPU box has no
-/root/reference) — with `inference_extensions_cuda` resolving to THIS repository's package and
+test_compress_time.py:23-69) are imported / executed as they are — from the sourceless byte-code `oracle/build_ref.py`
+emits into oracle/_ref/py — with `inference_extensions_cuda` resolving to THIS repository's package and
 `MLCodec_extensions_cpp` to the reference coder built into oracle/_ref.  Nothing of the reference is patched.
 
 Checks: the reference classes produce the same bytes and reconstructions as the repo's host-side mirrors
@@ -30,16 +29,13 @@ SKIP = 0.15
 
 
 def _ref_py_root():
-    if os.path.isdir("/root/reference/src/models"):
-        return "/root/reference", ".py"
-    p = os.path.join(ROOT, "baseline", "_ref", "py")
-    if os.path.isdir(os.path.join(p, "src", "models")):
-        return p, ".pyc"
-    return None, None
+    from oracle.build_ref import py_surface_root
+    p = py_surface_root()
+    return (p, ".pyc") if p else (None, None)
 
 
 REF_ROOT, REF_EXT = _ref_py_root()
-needs_ref = pytest.mark.skipif(REF_ROOT is None, reason="reference Python surface not built (python baseline/build_ref_cuda.py)")
+needs_ref = pytest.mark.skipif(REF_ROOT is None, reason="reference Python surface not built (python oracle/build_ref.py)")
 
 
 @pytest.fixture(scope="module")
