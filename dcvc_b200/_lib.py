@@ -68,6 +68,12 @@ SIGNATURES = {
     "dcvc_op_yuv420_to_frame": (C.c_int, [_P, _P, _P, _I, _I, _P, _L, _L, _L, _P]),
     "dcvc_op_frame_to_yuv420": (C.c_int, [_P, _L, _L, _L, _I, _I, _P, _P, _P, _P]),
     "dcvc_op_sse_u8": (C.c_int, [_P, _P, _L, _P, _P]),
+    "dcvc_op_rgb_to_frame": (C.c_int, [_P, _I, _I, _P, _L, _L, _L, _P]),
+    "dcvc_op_frame_to_rgb": (C.c_int, [_P, _L, _L, _L, _I, _I, _P, _P]),
+    "dcvc_op_metric_planes": (C.c_int, [_P, _L, _L, _L, _I, _I, _I, _P, _P]),
+    "dcvc_metrics_workspace_bytes": (C.c_int64, [_I, C.POINTER(_I)]),
+    "dcvc_op_metrics_sse": (C.c_int, [_I, C.POINTER(_I), C.POINTER(_P), C.POINTER(_P), _P, _P, _I, _P]),
+    "dcvc_op_msssim": (C.c_int, [_I, C.POINTER(_I), C.POINTER(_P), C.POINTER(_P), _P, _P, _I, _P]),
     "dcvc_op_square": (C.c_int, [C.POINTER(View), C.POINTER(View), _P]),
     "dcvc_op_warp_bilinear": (C.c_int, [C.POINTER(View), _P, _L, _L, _L, C.POINTER(View), _P]),
     "dcvc_op_int8_to_half": (C.c_int, [_P, _P, _L, _P]),

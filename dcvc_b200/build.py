@@ -23,6 +23,7 @@ SOURCES = [
     "dcb_tail.cu",
     "elementwise.cu",
     "frame_io.cu",
+    "metrics.cu",
     "family_ops.cu",
     "rans_host.cpp",
     "c_api_ops.cu",

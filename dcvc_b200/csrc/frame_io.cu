@@ -165,6 +165,126 @@ sse_u8_kernel(const uint8_t* __restrict__ a, const uint8_t* __restrict__ b, long
     if ((threadIdx.x & 31) == 0 && acc) atomicAdd(out, acc);
 }
 
+// ---- RGB sources (test_cfg/all_RGB.json: src_type == 'png') ----
+// BT.709 constants of src/utils/transforms.py:10-14 as torch applies them to fp32 tensors: a Python scalar becomes an
+// fp32 operand, and division by a scalar is a multiplication by its fp32 reciprocal (ATen's div_true CUDA kernel).
+// Every op rounds once: __fmul_rn / __fadd_rn keep nvcc from contracting them into FMAs.
+struct Bt709 {
+    float kr, kg, kb;
+    float inv255;        // x.float() / 255.0
+    float inv_1mkb;      // / (1 - Kb)
+    float inv_1mkr;      // / (1 - Kr)
+    float c2mkr, c2mkb;  // (2 - 2 * Kr), (2 - 2 * Kb)
+    float inv_kg;        // / Kg
+};
+
+static Bt709 bt709()
+{
+    const double Kr = 0.2126, Kg = 0.7152, Kb = 0.0722;
+    Bt709 c;
+    c.kr = static_cast<float>(Kr);
+    c.kg = static_cast<float>(Kg);
+    c.kb = static_cast<float>(Kb);
+    c.inv255 = 1.0f / static_cast<float>(255.0);
+    c.inv_1mkb = 1.0f / static_cast<float>(1 - Kb);
+    c.inv_1mkr = 1.0f / static_cast<float>(1 - Kr);
+    c.c2mkr = static_cast<float>(2 - 2 * Kr);
+    c.c2mkb = static_cast<float>(2 - 2 * Kb);
+    c.inv_kg = 1.0f / static_cast<float>(Kg);
+    return c;
+}
+
+__device__ __forceinline__ float clamp01(float v) { return fminf(fmaxf(v, 0.f), 1.f); }
+
+// rgb2ycbcr(x.float() / 255.0).half() - 0.5 (test_video.py:93-95, 115-122; transforms.py:17-27), one pixel per thread
+__global__ void __launch_bounds__(256)
+rgb_to_frame_kernel(const uint8_t* __restrict__ rgb, int H, int W, __half* __restrict__ x, long long sc, long long sh,
+                    long long sw, Bt709 k)
+{
+    const long long n = static_cast<long long>(H) * W;
+    const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int yy = static_cast<int>(i / W), xx = static_cast<int>(i % W);
+    const float r = __fmul_rn(static_cast<float>(rgb[i]), k.inv255);
+    const float g = __fmul_rn(static_cast<float>(rgb[n + i]), k.inv255);
+    const float b = __fmul_rn(static_cast<float>(rgb[2 * n + i]), k.inv255);
+    const float y = __fadd_rn(__fadd_rn(__fmul_rn(k.kr, r), __fmul_rn(k.kg, g)), __fmul_rn(k.kb, b));
+    const float cb = __fadd_rn(__fmul_rn(__fmul_rn(0.5f, __fsub_rn(b, y)), k.inv_1mkb), 0.5f);
+    const float cr = __fadd_rn(__fmul_rn(__fmul_rn(0.5f, __fsub_rn(r, y)), k.inv_1mkr), 0.5f);
+    __half* dst = x + yy * sh + xx * sw;
+    dst[0] = __float2half_rn(__half2float(__float2half_rn(clamp01(y))) - 0.5f);
+    dst[sc] = __float2half_rn(__half2float(__float2half_rn(clamp01(cb))) - 0.5f);
+    dst[2 * sc] = __float2half_rn(__half2float(__float2half_rn(clamp01(cr))) - 0.5f);
+}
+
+// ycbcr2rgb(x_hat + 0.5) (transforms.py:53-66): half -> fp32 math -> clamp -> half, per channel
+__device__ __forceinline__ void ycbcr_to_rgb_half(__half hy, __half hcb, __half hcr, const Bt709& k, __half out[3])
+{
+    const float y = __half2float(__float2half_rn(__half2float(hy) + 0.5f));
+    const float cb = __half2float(__float2half_rn(__half2float(hcb) + 0.5f));
+    const float cr = __half2float(__float2half_rn(__half2float(hcr) + 0.5f));
+    const float r = __fadd_rn(y, __fmul_rn(k.c2mkr, __fsub_rn(cr, 0.5f)));
+    const float b = __fadd_rn(y, __fmul_rn(k.c2mkb, __fsub_rn(cb, 0.5f)));
+    const float g = __fmul_rn(__fsub_rn(__fsub_rn(y, __fmul_rn(k.kr, r)), __fmul_rn(k.kb, b)), k.inv_kg);
+    out[0] = __float2half_rn(clamp01(r));
+    out[1] = __float2half_rn(clamp01(g));
+    out[2] = __float2half_rn(clamp01(b));
+}
+
+// x_hat[:, :, :H, :W] -> 8-bit planar RGB [3][H][W] as test_video.py:367-369 saves it:
+// clamp(ycbcr2rgb(x_hat + 0.5) * 255, 0, 255).round().byte(), every op in half
+__global__ void __launch_bounds__(256)
+frame_to_rgb_kernel(const __half* __restrict__ x, long long sc, long long sh, long long sw, int H, int W,
+                    uint8_t* __restrict__ rgb, Bt709 k)
+{
+    const long long n = static_cast<long long>(H) * W;
+    const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int yy = static_cast<int>(i / W), xx = static_cast<int>(i % W);
+    const __half* src = x + yy * sh + xx * sw;
+    __half c[3];
+    ycbcr_to_rgb_half(src[0], src[sc], src[2 * sc], k, c);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) rgb[j * n + i] = static_cast<uint8_t>(rintf(__half2float(to_255(c[j]))));
+}
+
+// ---- metric planes: the fp16 arrays get_distortion (test_video.py:32-66) hands to calc_psnr / calc_msssim ----
+// yuv420: Y [H][W] = clamp((x_hat + 0.5) * 255), then U, V [H/2][W/2] = the same after the 2x2 average;
+// rgb: [3][H][W] = clamp(ycbcr2rgb(x_hat + 0.5) * 255).  No rounding: these are frame_to_yuv420 / frame_to_rgb minus
+// their last step.  One thread per output pixel of Y (yuv420) or per pixel (rgb).
+template <bool RGB>
+__global__ void __launch_bounds__(256)
+metric_planes_kernel(const __half* __restrict__ x, long long sc, long long sh, long long sw, int H, int W,
+                     __half* __restrict__ rec, Bt709 k)
+{
+    const long long n = static_cast<long long>(H) * W;
+    const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int yy = static_cast<int>(i / W), xx = static_cast<int>(i % W);
+    const __half* src = x + yy * sh + xx * sw;
+    if (RGB) {
+        __half c[3];
+        ycbcr_to_rgb_half(src[0], src[sc], src[2 * sc], k, c);
+#pragma unroll
+        for (int j = 0; j < 3; ++j) rec[j * n + i] = to_255(c[j]);
+        return;
+    }
+    rec[i] = to_255(__float2half_rn(__half2float(src[0]) + 0.5f));
+    if ((yy & 1) || (xx & 1)) return;
+    const long long nc = n / 4;
+    const long long ci = static_cast<long long>(yy >> 1) * (W >> 1) + (xx >> 1);
+#pragma unroll
+    for (int ch = 1; ch <= 2; ++ch) {
+        float s = 0.f;   // avg_pool2d: fp32 sum in (0,0), (0,1), (1,0), (1,1) order, / 4, to half
+#pragma unroll
+        for (int r = 0; r < 2; ++r)
+#pragma unroll
+            for (int c = 0; c < 2; ++c)
+                s += __half2float(__float2half_rn(__half2float(src[r * sh + c * sw + ch * sc]) + 0.5f));
+        rec[n + (ch - 1) * nc + ci] = to_255(__float2half_rn(s / 4.f));
+    }
+}
+
 }  // namespace dcvc
 
 extern "C" {
@@ -214,6 +334,42 @@ int dcvc_op_sse_u8(const void* a, const void* b, int64_t n, void* sse_u64, void*
     if (blocks > 148 * 8) blocks = 148 * 8;
     dcvc::sse_u8_kernel<<<static_cast<int>(blocks), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const uint8_t*>(a), static_cast<const uint8_t*>(b), n, static_cast<unsigned long long*>(sse_u64));
+    return cudaGetLastError() == cudaSuccess ? 0 : 1;
+}
+
+int dcvc_op_rgb_to_frame(const void* rgb, int32_t H, int32_t W, void* x, int64_t sc, int64_t sh, int64_t sw, void* stream)
+{
+    if (H <= 0 || W <= 0) return 1;
+    static const dcvc::Bt709 k = dcvc::bt709();
+    const long long n = static_cast<long long>(H) * W;
+    dcvc::rgb_to_frame_kernel<<<dcvc::fio_blocks(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        static_cast<const uint8_t*>(rgb), H, W, static_cast<__half*>(x), sc, sh, sw, k);
+    return cudaGetLastError() == cudaSuccess ? 0 : 1;
+}
+
+int dcvc_op_frame_to_rgb(const void* x_hat, int64_t sc, int64_t sh, int64_t sw, int32_t H, int32_t W, void* rgb,
+                         void* stream)
+{
+    if (H <= 0 || W <= 0) return 1;
+    static const dcvc::Bt709 k = dcvc::bt709();
+    const long long n = static_cast<long long>(H) * W;
+    dcvc::frame_to_rgb_kernel<<<dcvc::fio_blocks(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        static_cast<const __half*>(x_hat), sc, sh, sw, H, W, static_cast<uint8_t*>(rgb), k);
+    return cudaGetLastError() == cudaSuccess ? 0 : 1;
+}
+
+int dcvc_op_metric_planes(const void* x_hat, int64_t sc, int64_t sh, int64_t sw, int32_t H, int32_t W, int32_t rgb,
+                          void* rec, void* stream)
+{
+    if (H <= 0 || W <= 0 || (!rgb && ((H & 1) || (W & 1)))) return 1;
+    static const dcvc::Bt709 k = dcvc::bt709();
+    const long long n = static_cast<long long>(H) * W;
+    if (rgb)
+        dcvc::metric_planes_kernel<true><<<dcvc::fio_blocks(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+            static_cast<const __half*>(x_hat), sc, sh, sw, H, W, static_cast<__half*>(rec), k);
+    else
+        dcvc::metric_planes_kernel<false><<<dcvc::fio_blocks(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+            static_cast<const __half*>(x_hat), sc, sh, sw, H, W, static_cast<__half*>(rec), k);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

@@ -118,6 +118,40 @@ int dcvc_op_frame_to_yuv420(const void* x_hat, int64_t sc, int64_t sh, int64_t s
 /* *sse_u64 += sum (a[i] - b[i])^2 over two 8-bit device arrays: the integer numerator of calc_psnr
  * (src/utils/metrics.py:10-24), so PSNR needs no frame on the host */
 int dcvc_op_sse_u8(const void* a, const void* b, int64_t n, void* sse_u64, void* stream);
+/* 8-bit planar RGB [3][H][W] (PNGReader.read_one_frame, device) -> fp16 model input channels 0..2 of x (element
+ * strides sc,sh,sw): rgb2ycbcr(x.float() / 255.0).half() - 0.5 (test_video.py:93-95, 115-122; BT.709,
+ * src/utils/transforms.py:17-27), bit-exact: fp32 ops rounded one at a time, division by a scalar as a multiplication
+ * by its fp32 reciprocal.  Any H, W. */
+int dcvc_op_rgb_to_frame(const void* rgb, int32_t H, int32_t W, void* x, int64_t sc, int64_t sh, int64_t sw,
+                         void* stream);
+/* fp16 reconstruction x_hat[:, :, :H, :W] -> 8-bit planar RGB [3][H][W] as the reference saves PNG frames
+ * (test_video.py:367-369: ycbcr2rgb(x_hat + 0.5) in fp32 with clamp (transforms.py:53-66), back to half, * 255,
+ * clamp, round half-to-even, byte()). */
+int dcvc_op_frame_to_rgb(const void* x_hat, int64_t sc, int64_t sh, int64_t sw, int32_t H, int32_t W, void* rgb,
+                         void* stream);
+
+/* ---- distortion metrics of test_video.py's per-job JSON (get_distortion, test_video.py:32-66) ----
+ * Metric planes: the unrounded fp16 arrays get_distortion measures, written to rec (fp16, contiguous):
+ * rgb == 0: Y [H][W] = clamp((x_hat + 0.5) * 255, 0, 255), then U, V [H/2][W/2] after the 2x2 chroma average
+ *           (yuv_444_to_420, transforms.py:83-90); H, W even;
+ * rgb != 0: [3][H][W] = clamp(ycbcr2rgb(x_hat + 0.5) * 255, 0, 255). */
+int dcvc_op_metric_planes(const void* x_hat, int64_t sc, int64_t sh, int64_t sw, int32_t H, int32_t W, int32_t rgb,
+                          void* rec, void* stream);
+/* Scratch for dcvc_op_metrics_sse / dcvc_op_msssim over nplanes (1..3) planes of sizes hw[2p] x hw[2p+1], in bytes
+ * (-1 on bad arguments).  One workspace serves both ops and every picture of that geometry. */
+int64_t dcvc_metrics_workspace_bytes(int32_t nplanes, const int32_t* hw);
+/* out[p * out_stride] = sum (src[p] - rec[p])^2 in fp64: calc_psnr's numerator (src/utils/metrics.py:10-24) for
+ * uint8 source planes and fp16 metric planes (contiguous rows).  Per-CTA partials + a fixed-order reduction:
+ * bitwise reproducible. */
+int dcvc_op_metrics_sse(int32_t nplanes, const int32_t* hw, const void* const* src, const void* const* rec,
+                        void* workspace, void* out, int32_t out_stride, void* stream);
+/* MS-SSIM levels of calc_msssim (src/utils/metrics.py:27-93) per plane pair: out[p * out_stride + 2l] and [.. + 2l + 1]
+ * = mean of the SSIM map and of the CS map at level l (11x11 Gaussian, sigma 1.5, 'valid' region, C1 = (0.01*255)^2,
+ * C2 = (0.03*255)^2; statistics and downsampled levels in fp64).  5 levels, 4 when a side is below 176; returns 2
+ * when a side is below 88 (the reference asserts).  The weighted product
+ * prod(mcs[:L-1] ** w[:L-1]) * mssim[L-1] ** w[L-1] is the caller's.  One launch per level + one; reproducible. */
+int dcvc_op_msssim(int32_t nplanes, const int32_t* hw, const void* const* src, const void* const* rec, void* workspace,
+                   void* out, int32_t out_stride, void* stream);
 
 /* ---- ops of the older DCVC-family codecs that north_star names (SURVEY.md §8 f4) ----
  * out = in * in, elementwise: the A operand of the GDN GEMM (gdn.py:58: F.conv2d(x ** 2, gamma, beta)) */
