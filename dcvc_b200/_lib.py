@@ -31,6 +31,11 @@ class DcbTailDesc(C.Structure):
                 ("qscale", C.c_void_p), ("shortcut", C.c_int32)]
 
 
+class RateEstimate(C.Structure):
+    _fields_ = [("y_q16", C.c_int64), ("z_q16", C.c_int64), ("y_symbols", C.c_int32), ("ec_parallel", C.c_int32),
+                ("bytes", C.c_int64)]
+
+
 class EntropyStep(C.Structure):
     _fields_ = [("H", C.c_int32), ("W", C.c_int32), ("G", C.c_int32), ("step", C.c_int32),
                 ("y", C.c_void_p), ("y_pitch", C.c_int32),
@@ -92,6 +97,7 @@ SIGNATURES = {
     "dcvc_rans_dec_z": (C.c_int, [_P, _P, _I, _I, _I]),
     "dcvc_rans_dec_y": (C.c_int, [_P, _P, _P, _I]),
     "dcvc_pmf_to_quantized_cdf": (C.c_int, [_P, _I, _P]),
+    "dcvc_rans_cost_table": (C.c_int, [_P, _P, _I, _I, _P]),
     "dcvc_create": (C.c_int, [_I, _I, C.POINTER(_P)]),
     "dcvc_destroy": (C.c_int, [_P]),
     "dcvc_codec_error": (C.c_char_p, [_P]),
@@ -104,6 +110,7 @@ SIGNATURES = {
     "dcvc_compress_chunk": (C.c_int, [_P, _P, _I, _I, _L, _L, _L, _I, _I, _I, _I, _P, C.POINTER(_P),
                                       C.POINTER(_I), C.POINTER(_I)]),
     "dcvc_decompress_chunk": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _P, C.POINTER(_P)]),
+    "dcvc_estimate_bits": (C.c_int, [_P, _P, _I, _I, _L, _L, _L, _P, _I, _I, _I, _I, _P, C.POINTER(RateEstimate)]),
     "dcvc_kernel_launches": (C.c_int64, [_P]),
     "dcvc_last_gpu_ms": (C.c_int, [_P, C.POINTER(C.c_float)]),
     "dcvc_profile_enable": (C.c_int, [_P, _I]),

@@ -24,6 +24,7 @@ SOURCES = [
     "elementwise.cu",
     "frame_io.cu",
     "metrics.cu",
+    "rate.cu",
     "family_ops.cu",
     "rans_host.cpp",
     "c_api_ops.cu",

@@ -2,6 +2,7 @@
 #include <string.h>
 
 #include <memory>
+#include <stdexcept>
 #include <string>
 #include <vector>
 
@@ -328,6 +329,16 @@ int dcvc_pmf_to_quantized_cdf(const float* pmf, int32_t n, uint32_t* cdf_out)
     API_TRY
     std::vector<uint32_t> c = pmf_to_quantized_cdf(pmf, n);
     memcpy(cdf_out, c.data(), c.size() * sizeof(uint32_t));
+    return 0;
+    API_CATCH
+}
+
+int dcvc_rans_cost_table(const int32_t* cdf, const int32_t* cdf_sizes, int32_t rows, int32_t width, uint32_t* out)
+{
+    API_TRY
+    if (rows < 1 || width < 2) throw std::runtime_error("rans_cost_table: bad table shape");
+    std::vector<uint32_t> c = rans_cost_table(cdf, cdf_sizes, rows, width);
+    memcpy(out, c.data(), c.size() * sizeof(uint32_t));
     return 0;
     API_CATCH
 }

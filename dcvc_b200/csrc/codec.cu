@@ -33,6 +33,8 @@ public:
                   int32_t* ec_parallel, void* x_hat_out);
     void decompress(const uint8_t* bs, int len, int qp, int height, int width, int ec_parallel,
                     cudaStream_t stream, void* x_hat_out);
+    void estimate(const void* x, int H, int W, int64_t sc, int64_t sh, int64_t sw, const int32_t* qps, int n_qps,
+                  int pad_b, int pad_r, cudaStream_t stream, dcvc_rate_estimate* out) override;
     int debug_fetch(const char* name, void* dst, int64_t max_bytes, int64_t* written) override;
     int arena_overflow_blocks() const override { return arena_.overflow_blocks(); }
 
@@ -432,6 +434,33 @@ void IntraCodec::compress(const void* x, int H, int W, int64_t sc, int64_t sh, i
     *ec_parallel = n_par;
 }
 
+// =============================================================================== estimate
+// enc0 writes in8_, y_, the scratch levels, hyper / prior buffers, cat_, yhat_, z_i8_ and the symbol buffers, all of which
+// compress() and decompress() rewrite before they read them; x_hat comes from enc1 / dec4, which do not run here.
+void IntraCodec::estimate(const void* x, int H, int W, int64_t sc, int64_t sh, int64_t sw, const int32_t* qps, int n_qps,
+                          int pad_b, int pad_r, cudaStream_t stream, dcvc_rate_estimate* out)
+{
+    CK(cudaSetDevice(device_));
+    if ((H + pad_b) % 16 || (W + pad_r) % 16) throw std::runtime_error("padded size must be a multiple of 16");
+    check_rate_qps(qps, n_qps);
+    plan(H + pad_b, W + pad_r);
+    StreamHop hop(this, stream);
+    stream = hop.run;
+    if (launch_unshuffle8_pad(static_cast<const __half*>(x), 3, H, W, sc, sh, sw,
+                              make_view(in8_, kChSrc, kChSrc, W8_, H8_), stream))
+        throw std::runtime_error("unshuffle8_pad launch failed");
+    ++launches;
+    const int16_t* ys[4] = { sym_c_[0], sym_c_[1], sym_c_[2], sym_c_[3] };
+    const int32_t* counts[4] = { totals_, totals_ + 1, totals_ + 2, totals_ + 3 };
+    const int nz = H64_ * W64_ * kChZ;
+    for (int i = 0; i < n_qps; ++i) {
+        stage_qp(qps[i], stream);
+        run(enc0_, stream);
+        rate_trial(ys, counts, 4, quarter_, z_i8_, nz, qps[i], i, stream);
+    }
+    rate_finish(n_qps, stream, out);
+}
+
 // =============================================================================== decompress
 void IntraCodec::decompress(const uint8_t* bs, int len, int qp, int height, int width,
                             int ec_parallel, cudaStream_t stream, void* x_hat_out)
@@ -729,6 +758,17 @@ int dcvc_decompress_chunk(dcvc_codec* h, const uint8_t* bit_stream, int32_t len,
     if (h->kind != DCVC_KIND_HTS) throw std::runtime_error("decompress_chunk needs a video codec handle");
     return dcvc::hts_decompress(h->base.get(), bit_stream, len, qp, height, width, ec_parallel, reset_feature_memory,
                                 static_cast<cudaStream_t>(stream), x_hat_out);
+    CODEC_CATCH(h)
+}
+
+int dcvc_estimate_bits(dcvc_codec* h, const void* x, int32_t H, int32_t W, int64_t sc, int64_t sh, int64_t sw,
+                       const int32_t* qps, int32_t n_qps, int32_t reset_feature_memory, int32_t pad_b, int32_t pad_r,
+                       void* stream, dcvc_rate_estimate* out)
+{
+    CODEC_TRY(h)
+    (void)reset_feature_memory;   // selects the memory update after the unit, which the estimate does not run
+    h->base->estimate(x, H, W, sc, sh, sw, qps, n_qps, pad_b, pad_r, static_cast<cudaStream_t>(stream), out);
+    return 0;
     CODEC_CATCH(h)
 }
 

@@ -24,10 +24,13 @@
 #include "elementwise.cuh"
 #include "pw_gemm.cuh"
 #include "rans_host.h"
+#include "rate.cuh"
 
 namespace dcvc {
 
 constexpr int kQpNum = 64;
+constexpr int kMaxRateTrials = 64;   // QPs per dcvc_estimate_bits call
+constexpr int kRateZCh = 128;        // z channels of every codec kind: CDF row = k % 128 + qp * 128
 
 #define CK(expr)                                                                           \
     do {                                                                                   \
@@ -229,6 +232,7 @@ public:
     {
         if (copy_stream_) cudaStreamDestroy(copy_stream_);
         if (own_stream_) cudaStreamDestroy(own_stream_);
+        if (h_rate_slots_) cudaFreeHost(h_rate_slots_);
         if (ev_hop_) cudaEventDestroy(ev_hop_);
         if (ev_y_) cudaEventDestroy(ev_y_);
         if (ev_fork_) cudaEventDestroy(ev_fork_);
@@ -241,6 +245,10 @@ public:
 
     virtual void finalize(float skip_thres) = 0;
     virtual int debug_fetch(const char* name, void* dst, int64_t max_bytes, int64_t* written) = 0;
+    // dcvc_estimate_bits: the unit's size at each QP from the analysis graph and the rate kernel alone (no synthesis,
+    // no feature-memory update, no rANS).  Leaves every buffer a later compress() reads as it found it.
+    virtual void estimate(const void* x, int H, int W, int64_t sc, int64_t sh, int64_t sw, const int32_t* qps, int n_qps,
+                          int pad_b, int pad_r, cudaStream_t stream, dcvc_rate_estimate* out) = 0;
     virtual int arena_overflow_blocks() const { return 0; }   // > 0: the plan's arena estimate was short (tests)
 
     void set_param(const char* name, const void* data, int dtype, int ndim, const int64_t* shape, int on_device)
@@ -402,9 +410,23 @@ protected:
             const HostTensor& l = param(std::string(names[i]) + "cdf_length");
             if (c.dtype != DCVC_DTYPE_I32 || l.dtype != DCVC_DTYPE_I32 || c.shape.size() != 2)
                 throw std::runtime_error("CDF tables must be int32 [rows][width]");
-            rans_.set_cdf(reinterpret_cast<const int32_t*>(c.bytes.data()), reinterpret_cast<const int32_t*>(l.bytes.data()),
-                          static_cast<int>(c.shape[0]), static_cast<int>(c.shape[1]), i);
+            const int32_t* cdf = reinterpret_cast<const int32_t*>(c.bytes.data());
+            const int32_t* len = reinterpret_cast<const int32_t*>(l.bytes.data());
+            const int rows = static_cast<int>(c.shape[0]), width = static_cast<int>(c.shape[1]);
+            rans_.set_cdf(cdf, len, rows, width, i);
+            // the rate estimate's code-length table and escape symbols of this set (rate.cu)
+            const std::vector<uint32_t> cost = rans_cost_table(cdf, len, rows, width);
+            std::vector<int8_t> maxv(rows);
+            for (int r = 0; r < rows; ++r) maxv[r] = static_cast<int8_t>(len[r] - 2);
+            cost_[i] = static_cast<uint32_t*>(warena_.alloc(cost.size() * 4));
+            maxv_[i] = static_cast<int8_t*>(warena_.alloc(rows));
+            CK(cudaMemcpy(cost_[i], cost.data(), cost.size() * 4, cudaMemcpyHostToDevice));
+            CK(cudaMemcpy(maxv_[i], maxv.data(), rows, cudaMemcpyHostToDevice));
+            cost_rows_[i] = rows;
+            cost_width_[i] = width;
         }
+        rate_slots_ = static_cast<RateSlot*>(warena_.alloc(sizeof(RateSlot) * kMaxRateTrials));
+        if (!h_rate_slots_) CK(cudaMallocHost(&h_rate_slots_, sizeof(RateSlot) * kMaxRateTrials));
         if (!copy_stream_) {
             int lo, hi;
             CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
@@ -699,6 +721,48 @@ protected:
         launches += s.launches;
     }
 
+    // ------------------------------------------------------------------ rate estimate (rate.cu)
+    static void check_rate_qps(const int32_t* qps, int n)
+    {
+        if (n < 1 || n > kMaxRateTrials) throw std::runtime_error("estimate_bits: between 1 and 64 QPs per call");
+        for (int i = 0; i < n; ++i)
+            if (qps[i] < 0 || qps[i] >= kQpNum) throw std::runtime_error("qp out of range");
+    }
+    // after enc0 at `qp`: the rate kernel over the y steps and z into result slot `slot`
+    void rate_trial(const int16_t* const* y, const int32_t* const* counts, int n_y, size_t y_capacity, const int8_t* z,
+                    int nz, int qp, int slot, cudaStream_t stream)
+    {
+        RateArgs a{};
+        for (int k = 0; k < n_y; ++k) { a.y[k] = y[k]; a.y_count[k] = counts[k]; }
+        a.n_y = n_y;
+        a.z = z; a.nz = nz; a.z_ch = kRateZCh; a.z_row0 = qp * kRateZCh;
+        a.y_cost = cost_[1]; a.y_maxv = maxv_[1]; a.y_rows = cost_rows_[1]; a.y_width = cost_width_[1];
+        a.z_cost = cost_[0]; a.z_maxv = maxv_[0]; a.z_width = cost_width_[0];
+        a.out = rate_slots_ + slot;
+        if (a.z_row0 + kRateZCh > cost_rows_[0]) throw std::runtime_error("estimate_bits: the z CDF table has no rows for this qp");
+        if (!rate_smem_bytes(a.y_rows, a.y_width, a.z_ch, a.z_width)) throw std::runtime_error("estimate_bits: CDF tables too large");
+        if (launch_rate_estimate(a, y_capacity, stream)) throw std::runtime_error("rate_estimate launch failed");
+        ++launches;
+    }
+    // one copy of the slots, one synchronise; bytes = the coded symbols + 4 flush bytes per rANS stream + the offset
+    // words of the merged container (RansCodec::encode)
+    void rate_finish(int n, cudaStream_t stream, dcvc_rate_estimate* out)
+    {
+        CK(cudaMemcpyAsync(h_rate_slots_, rate_slots_, sizeof(RateSlot) * n, cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        for (int i = 0; i < n; ++i) {
+            const RateSlot& s = h_rate_slots_[i];
+            const int ec = RansCodec::ec_parallel_for(s.y_symbols);
+            const int n_off = ec / 2 - 1 + ec % 2;
+            out[i].y_q16 = static_cast<int64_t>(s.y_q16);
+            out[i].z_q16 = static_cast<int64_t>(s.z_q16);
+            out[i].y_symbols = s.y_symbols;
+            out[i].ec_parallel = ec;
+            const uint64_t q16 = s.y_q16 + s.z_q16;
+            out[i].bytes = static_cast<int64_t>((q16 + (8ull << 16) - 1) / (8ull << 16)) + 4 * ec + 4 * n_off;
+        }
+    }
+
     void tick(cudaStream_t st)
     {
         if (tev_n_ + 2 <= static_cast<int>(tev_.size())) CK(cudaEventRecord(tev_[tev_n_], st));
@@ -763,6 +827,12 @@ protected:
     std::vector<cudaEvent_t> prof_events_;
     int tev_n_ = 0;
     std::vector<uint8_t> bitstream_;
+    // rate estimate: Q16 code lengths and escape symbols of CDF set 0 (z) and 1 (y), one device slot per QP trial
+    uint32_t* cost_[2] = { nullptr, nullptr };
+    int8_t* maxv_[2] = { nullptr, nullptr };
+    int cost_rows_[2] = { 0, 0 }, cost_width_[2] = { 0, 0 };
+    RateSlot* rate_slots_ = nullptr;
+    RateSlot* h_rate_slots_ = nullptr;
 };
 
 }  // namespace dcvc

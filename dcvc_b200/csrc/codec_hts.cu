@@ -30,6 +30,8 @@ public:
                   int pad_r, cudaStream_t stream, const uint8_t** bs, int32_t* len, int32_t* ec);
     void decompress(const uint8_t* bs, int len, int qp, int height, int width, int ec, int reset,
                     cudaStream_t stream, void* const* x_hat_out);
+    void estimate(const void* x, int H, int W, int64_t sc, int64_t sh, int64_t sw, const int32_t* qps, int n_qps,
+                  int pad_b, int pad_r, cudaStream_t stream, dcvc_rate_estimate* out) override;
 
 private:
     void plan(int height, int width);
@@ -500,6 +502,33 @@ void HtsCodec::compress(const void* x, int H, int W, int64_t sc, int64_t sh, int
     *bs = bitstream_.data();
     *len = static_cast<int32_t>(bitstream_.size());
     *ec = n_par;
+}
+
+// =============================================================================== estimate
+// The unshuffle fills only the source channels of cat_enc_ (its context channels come from the previous unit's s_fe_),
+// and enc0 reads the feature memory without writing it; everything else enc0 writes, compress() and decompress()
+// rewrite before they read.  So the state the next unit is coded from is untouched.
+void HtsCodec::estimate(const void* x, int H, int W, int64_t sc, int64_t sh, int64_t sw, const int32_t* qps, int n_qps,
+                        int pad_b, int pad_r, cudaStream_t stream, dcvc_rate_estimate* out)
+{
+    CK(cudaSetDevice(device_));
+    if ((H + pad_b) % 16 || (W + pad_r) % 16) throw std::runtime_error("padded size must be a multiple of 16");
+    check_rate_qps(qps, n_qps);
+    plan(H + pad_b, W + pad_r);
+    StreamHop hop(this, stream);
+    stream = hop.run;
+    if (launch_unshuffle8_pad(static_cast<const __half*>(x), 3 * kG, H, W, sc, sh, sw, make_view(cat_enc_, kSrcD, 2048, W8_, H8_), stream))
+        throw std::runtime_error("unshuffle8_pad launch failed");
+    ++launches;
+    const int16_t* ys[1] = { sym_c_ };
+    const int32_t* counts[1] = { total_ };
+    const int nz = H64_ * W64_ * kZ;
+    for (int i = 0; i < n_qps; ++i) {
+        stage_qp(qps[i], stream);
+        run(s_enc0_, stream);
+        rate_trial(ys, counts, 1, n_lat_, z_i8_, nz, qps[i], i, stream);
+    }
+    rate_finish(n_qps, stream, out);
 }
 
 // =============================================================================== decompress

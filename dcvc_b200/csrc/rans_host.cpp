@@ -8,6 +8,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <numeric>
 #include <stdexcept>
 
@@ -546,6 +547,21 @@ std::vector<uint32_t> pmf_to_quantized_cdf(const float* pmf, int n)
         }
     }
     return cdf;
+}
+
+std::vector<uint32_t> rans_cost_table(const int32_t* cdf, const int32_t* cdf_sizes, int rows, int width)
+{
+    std::vector<uint32_t> out(static_cast<size_t>(rows) * width, 0u);
+    for (int r = 0; r < rows; ++r) {
+        const int32_t* c = cdf + static_cast<size_t>(r) * width;
+        const int maxv = std::min(cdf_sizes[r] - 2, width - 2);
+        for (int s = 0; s <= maxv; ++s) {
+            const int32_t freq = std::max(c[s + 1] - c[s], 1);   // a valid table has no zero-width symbol
+            out[static_cast<size_t>(r) * width + s] =
+                static_cast<uint32_t>(std::llround(65536.0 * (kScaleBits - std::log2(static_cast<double>(freq)))));
+        }
+    }
+    return out;
 }
 
 }  // namespace dcvc

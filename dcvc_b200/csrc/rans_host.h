@@ -92,4 +92,8 @@ private:
 // ryg-style pmf -> 16-bit quantised cdf (py_rans.cpp:36-94)
 std::vector<uint32_t> pmf_to_quantized_cdf(const float* pmf, int n);
 
+// Code lengths of one CDF set in Q16 bits, [rows][width] like the CDF: entry s of row r (s <= cdf_sizes[r] - 2) is
+// round(65536 * (16 - log2(cdf[s + 1] - cdf[s]))), what enc_symbol spends on that symbol; the other entries are 0.
+std::vector<uint32_t> rans_cost_table(const int32_t* cdf, const int32_t* cdf_sizes, int rows, int width);
+
 }  // namespace dcvc

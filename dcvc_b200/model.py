@@ -100,6 +100,11 @@ class DMCI:
         bit_stream, x_hat, ec_parallel = self.proxy.compress(x, qp, padding_b, padding_r)
         return {"bit_stream": bit_stream.tobytes(), "x_hat": x_hat, "ec_parallel": ec_parallel}
 
+    def estimate_bits(self, x, qps, padding_b, padding_r):
+        """compress()'s size at each QP of `qps` without coding: one dict per QP (bits_y, bits_z, ec_parallel, bytes, ...)"""
+        self._ensure_proxy()
+        return self.proxy.estimate_bits(x, qps, padding_b, padding_r)
+
     def decompress(self, bit_stream, sps, qp, ec_part):
         self._ensure_proxy()   # the reference needs a prior compress(); we tolerate decode-first use
         x_hat = self.proxy.decompress(np.frombuffer(bit_stream, dtype=np.uint8), qp, sps["height"], sps["width"],
@@ -151,6 +156,13 @@ class DMC(DMCI):
         self._check_dpb()
         bit_stream, ec_parallel = self.proxy.compress(x, qp, reset_feature_memory, padding_b, padding_r)
         return {"bit_stream": bit_stream.tobytes(), "ec_parallel": ec_parallel}
+
+    def estimate_bits(self, x, qps, reset_feature_memory, padding_b, padding_r):
+        """compress()'s size at each QP of `qps` without coding (see DMCI.estimate_bits); needs the same reference as
+        compress()"""
+        self._ensure_proxy()
+        self._check_dpb()
+        return self.proxy.estimate_bits(x, qps, reset_feature_memory, padding_b, padding_r)
 
     def decompress(self, bit_stream, sps, qp, ec_part, reset_feature_memory):
         self._ensure_proxy()

@@ -75,6 +75,21 @@ def _push_state_dict(hd: _CodecHandle, state_dict, skip_threshold: float):
     hd.check(hd.lib.dcvc_finalize_params(hd.h, C.c_float(float(skip_threshold))), "finalize_params")
 
 
+def _estimate_bits(hd: _CodecHandle, x, qps, reset_feature_memory, padding_b, padding_r):
+    """dcvc_estimate_bits: one record per QP, in the order given"""
+    qps = [int(q) for q in qps]
+    hd.same_device(x)
+    _, _, H, W = x.shape
+    q = (C.c_int32 * len(qps))(*qps)
+    res = (_lib.RateEstimate * len(qps))()
+    stream = C.c_void_p(torch.cuda.current_stream(hd.device).cuda_stream)
+    hd.check(hd.lib.dcvc_estimate_bits(hd.h, C.c_void_p(x.data_ptr()), H, W, x.stride(1), x.stride(2), x.stride(3), q,
+                                       len(qps), 1 if reset_feature_memory else 0, int(padding_b), int(padding_r), stream,
+                                       res), "estimate_bits")
+    return [{"qp": qp, "bits_y": r.y_q16 / 65536.0, "bits_z": r.z_q16 / 65536.0, "y_symbols": r.y_symbols,
+             "ec_parallel": r.ec_parallel, "bytes": r.bytes} for qp, r in zip(qps, res)]
+
+
 class DMCIProxy:
     """DCVC-UF-Intra proxy (reference: DMCIProxy, dmci_proxy.h:142-144)."""
 
@@ -110,6 +125,13 @@ class DMCIProxy:
                                       C.byref(ec), C.c_void_p(out.data_ptr())), "compress")
         stream_np = np.ctypeslib.as_array(C.cast(bs, C.POINTER(C.c_uint8)), (n.value,)).copy()
         return stream_np, out, ec.value
+
+    def estimate_bits(self, x: torch.Tensor, qps, padding_b: int, padding_r: int):
+        """Size of compress(x, qp, ...) for each qp in `qps` without coding it: a list of dicts with bits_y / bits_z
+        (the y and z symbols' code lengths, exact in Q16), y_symbols, ec_parallel and bytes (the stream length to within
+        a few bytes per rANS stream).  Runs the analysis graph per QP and changes no state of the proxy."""
+        assert x.is_cuda and x.dtype == torch.float16 and x.dim() == 4 and x.shape[0] == 1 and x.shape[1] == 3
+        return _estimate_bits(self._hd, x, qps, False, padding_b, padding_r)
 
     def decompress(self, bit_stream: np.ndarray, qp: int, height: int, width: int, ec_parallel: int):
         """-> x_hat: fp16 channels_last [1,3,H16p,W16p], a proxy-owned buffer reused by the next decompress() call"""
@@ -186,6 +208,13 @@ class DMCHTSProxy:
                                             int(qp), 1 if reset_feature_memory else 0, int(padding_b), int(padding_r),
                                             stream, C.byref(bs), C.byref(n), C.byref(ec)), "compress")
         return np.ctypeslib.as_array(C.cast(bs, C.POINTER(C.c_uint8)), (n.value,)).copy(), ec.value
+
+    def estimate_bits(self, x: torch.Tensor, qps, reset_feature_memory: bool, padding_b: int, padding_r: int):
+        """Size of compress(x, qp, reset_feature_memory, ...) for each qp in `qps` without coding it (see
+        DMCIProxy.estimate_bits).  The feature memory, context and every other state the next compress() reads stay
+        as they were."""
+        assert x.is_cuda and x.dtype == torch.float16 and x.dim() == 4 and x.shape[1] == 3 * self.FRAMES
+        return _estimate_bits(self._hd, x, qps, reset_feature_memory, padding_b, padding_r)
 
     def decompress(self, bit_stream: np.ndarray, qp: int, height: int, width: int, ec_parallel: int,
                    reset_feature_memory: bool):

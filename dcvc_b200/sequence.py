@@ -129,9 +129,11 @@ def _converters(src_type: str):
 class SequenceEncoder:
     def __init__(self, i_net, p_net, height: int, width: int, qp_i: int, qp_p: int, frame_delay: int = 8,
                  intra_period: int = -1, reset_interval: int = 32, force_intra: bool = False,
-                 to_model: Optional[Callable] = None, src_type: str = "yuv420"):
+                 to_model: Optional[Callable] = None, src_type: str = "yuv420", rate_control=None):
         self.i_net, self.p_net = i_net, p_net
         self.src_type = src_type
+        # rate_control: a dcvc_b200.rate_control.RateController; each unit's QP then comes from it (qp_i / qp_p unused)
+        self.rate_control = rate_control
         self.height, self.width = height, width
         self.qp_i, self.qp_p = qp_i, qp_p
         self.frame_delay, self.intra_period, self.reset_interval = frame_delay, intra_period, reset_interval
@@ -154,14 +156,22 @@ class SequenceEncoder:
             x = self.to_model(group, self.frame_delay)
             if self.timer:
                 self.timer.start()
+            rc = self.rate_control
             if unit.is_intra:
                 qp = self.qp_i
+                if rc is not None:
+                    qp = rc.choose(unit.first, unit.count, True, lambda qps: [
+                        r["bytes"] for r in self.i_net.estimate_bits(x, qps, self.padding_b, self.padding_r)])
                 encoded = self.i_net.compress(x, qp, self.padding_b, self.padding_r)
                 if not self.force_intra:
                     self.p_net.clear_dpb()
                     self.p_net.add_ref_feature_from_frame(encoded["x_hat"])
             else:
                 qp = self.qp_p
+                if rc is not None:
+                    qp = rc.choose(unit.first, unit.count, False, lambda qps: [
+                        r["bytes"] for r in self.p_net.estimate_bits(x, qps, unit.reset_feature_memory, self.padding_b,
+                                                                     self.padding_r)])
                 encoded = self.p_net.compress(x, qp, unit.reset_feature_memory, self.padding_b, self.padding_r)
             sps = {"sps_id": -1, "height": self.height, "width": self.width}
             sps_id, is_new = sps_helper.get_sps_id(sps)
@@ -170,6 +180,8 @@ class SequenceEncoder:
             n += write_ip(out, unit.is_intra, sps_id, qp, encoded["ec_parallel"], unit.reset_feature_memory,
                           encoded["bit_stream"])
             self.bits += [n * 8] + [0] * (unit.count - 1)
+            if rc is not None:
+                rc.update(n)
             if self.timer:
                 self.unit_ms.append(self.timer.stop())
         return out.getvalue()
@@ -226,7 +238,7 @@ TIME_BYPASS_UNITS = 4      # test_video.py:376-377: the first 4 coded units are 
 def run_job(i_net, p_net, frames: Sequence, height: int, width: int, qp_i: int, qp_p: int, frame_delay: int = 8,
             intra_period: int = -1, reset_interval: int = 32, src_type: str = "yuv420", calc_ssim: bool = False,
             verbose_json: bool = False, verbose: int = 0, to_model: Optional[Callable] = None,
-            metrics: Optional[Callable] = None, timer: Optional[Callable] = None):
+            metrics: Optional[Callable] = None, timer: Optional[Callable] = None, rate_control=None):
     """One job of test_video.py (run_one_point_with_stream, test_video.py:166-398): encode `frames`, decode the
     stream, measure every decoded picture against its source, and build the per-job record.
 
@@ -238,7 +250,10 @@ def run_job(i_net, p_net, frames: Sequence, height: int, width: int, qp_i: int, 
     4 units are reported in seconds, as the reference does.  Distortion is computed outside the timed regions.
 
     Injection points for tests: `to_model` (source frames -> model tensor), `metrics` (a factory with Distortion's
-    signature and .add / .results), `timer` (a factory of objects with .start() / .stop() -> ms)."""
+    signature and .add / .results), `timer` (a factory of objects with .start() / .stop() -> ms).
+
+    `rate_control` (a dcvc_b200.rate_control.RateController) chooses every unit's QP instead of qp_i / qp_p; its size
+    trials run inside the unit's timed region, as encoding time."""
     import time
 
     if metrics is None:
@@ -249,7 +264,7 @@ def run_job(i_net, p_net, frames: Sequence, height: int, width: int, qp_i: int, 
     timer = timer or UnitTimer
     start_time = time.time()
     enc = SequenceEncoder(i_net, p_net, height, width, qp_i, qp_p, frame_delay, intra_period, reset_interval,
-                          to_model=to_model, src_type=src_type)
+                          to_model=to_model, src_type=src_type, rate_control=rate_control)
     enc.timer = timer()
     data = enc.encode(frames)
     frame_types: List[int] = []

@@ -210,6 +210,9 @@ int dcvc_rans_dec_set_stream(dcvc_rans* r, const uint8_t* data, int32_t size, in
 int dcvc_rans_dec_z(dcvc_rans* r, int8_t* out, int32_t n, int32_t cdf_offset, int32_t ch);
 int dcvc_rans_dec_y(dcvc_rans* r, int8_t* out, const uint8_t* cdf_rows, int32_t n);
 int dcvc_pmf_to_quantized_cdf(const float* pmf, int32_t n, uint32_t* cdf_out /* n+1 */);
+/* code lengths of a CDF set in Q16 bits, out = uint32 [rows][width]: entry s of row r (s <= cdf_sizes[r] - 2) is
+ * round(65536 * (16 - log2(cdf[r][s+1] - cdf[r][s]))), the rest 0.  The table dcvc_estimate_bits sums on the device. */
+int dcvc_rans_cost_table(const int32_t* cdf, const int32_t* cdf_sizes, int32_t rows, int32_t width, uint32_t* out);
 
 /* ---------------------------------------------------------------------------------------------
  * Codec-level ABI — what the pybind classes DMCIProxy / DMCHTSProxy bind (bind.cpp:13-31).
@@ -256,6 +259,22 @@ int dcvc_compress_chunk(dcvc_codec* h, const void* x, int32_t H, int32_t W, int6
 int dcvc_decompress_chunk(dcvc_codec* h, const uint8_t* bit_stream, int32_t len, int32_t qp,
                           int32_t height, int32_t width, int32_t ec_parallel,
                           int32_t reset_feature_memory, void* stream, void* const* x_hat_out);
+
+/* Rate estimate of one coded unit at each of n_qps QPs (1..64), for rate control.  x, H, W, strides and padding as for
+ * dcvc_compress (Intra, LD) / dcvc_compress_chunk (HT-S, HT-L); reset_feature_memory does not change the estimate (it
+ * only selects the memory update after the unit) and is ignored for Intra.  Runs the analysis graph and an integer
+ * reduction of the symbols' code lengths on the device per QP, one copy and one synchronise at the end; no synthesis,
+ * no feature-memory update, no rANS, and the next compress gives the same bytes as without the call.
+ * y_q16 / z_q16: bits of the y / z symbols in Q16; ec_parallel: the stream count compress would use;
+ * bytes = ceil((y_q16 + z_q16) / 2^19) + 4 * ec_parallel + 4 * (offset words of the merged container). */
+typedef struct dcvc_rate_estimate {
+    int64_t y_q16, z_q16;
+    int32_t y_symbols, ec_parallel;
+    int64_t bytes;
+} dcvc_rate_estimate;
+int dcvc_estimate_bits(dcvc_codec* h, const void* x, int32_t H, int32_t W, int64_t sc, int64_t sh, int64_t sw,
+                       const int32_t* qps, int32_t n_qps, int32_t reset_feature_memory, int32_t pad_b, int32_t pad_r,
+                       void* stream, dcvc_rate_estimate* out);
 
 /* instrumentation for bench.py: kernels launched by this handle since creation, and the GPU-only
  * duration (ms) of the segments of the last compress/decompress (CUDA events on `stream`). */
